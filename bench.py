@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- Msamples/s (pixels x spp) of the volumetric render pass, BASELINE.json's metric.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config C]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config C] [--dump-outputs DIR]
 
 Default workload (the one the metric is quoted on): BASELINE.json configs[1] -- dragon.vdb, 1920x1080, 64 spp per step,
 ray_depth 100, volume_depth 1, direct integrator, sun + HDRI environment: 132.7 M samples per step.  `--config 1|3|4|5`
@@ -175,6 +175,14 @@ def timed_steps(step_fn, steps, warmup, dist, flush_buf, sampler=None):
     return ms, wall
 
 
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: what the timed path computed in its last step, one float32 .npy per array (34 MB at 1920x1080), so
+    that two builds run with the same arguments (hence the same inputs) can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy().astype(np.float32))
+
+
 def cpu_baseline_sample(V, scene, cam, kp, width, height, seconds_target=12.0):
     """CPU restatement (oracle/vpt_oracle.c, 'port') timed on the host cores over a bounded sample of the same workload."""
     try:
@@ -209,6 +217,8 @@ def main():
                     "Driver API exactly like the reference kernel (one launch + synchronize per spp), instead of the wavefront library")
     ap.add_argument("--cells", action="store_true", help="config 4: trace from the cell table (8 corner texels per cell = one 32-byte sector per look-up, software filter) instead of the 3-D texture")
     ap.add_argument("--fast", action="store_true", help="config 4: trace from the brick pool (TMA-staged software sampler) instead of the 3-D texture")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's frame (accum, depth) and blue-noise "
+                    "state as DIR/<name>.npy (float32)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -264,6 +274,8 @@ def main():
         sampler.start()
         ms, wall = timed_steps(step, args.steps, args.warmup, None, flush_buf, sampler)
         clocks = sampler.stop()
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"accum": r.buffers.accum, "depth": r.buffers.depth, "blue_noise": scene.d_blue_noise})
         val = samples_per_step * args.steps / (ms * 1e-3) / 1e6
         config.update({"launch_protocol": "reference main loop: 1 launch + cudaDeviceSynchronize per spp, grid (W/16+1,H/16+1)x(16,16)",
                        "kernel": kernel_note,
@@ -322,6 +334,12 @@ def main():
     sampler.start()
     ms, wall = timed_steps(step, args.steps, args.warmup, dist, flush_buf, sampler)
     clocks = sampler.stop()
+    if args.dump_outputs:
+        if world > 1:
+            full = dr.full_accum().reshape(-1, 3)          # the gathered frame; depth and blue noise stay rank-local
+            if rank == 0: dump_outputs(args.dump_outputs, {"accum": full})
+        else:
+            dump_outputs(args.dump_outputs, {"accum": r.buffers.accum, "depth": r.buffers.depth, "blue_noise": scene.d_blue_noise})
     l1, _ = r.stats()
     launches_per_step = (l1 - l0) // (args.steps + args.warmup)
     value = samples_per_step * args.steps / (ms * 1e-3) / 1e6

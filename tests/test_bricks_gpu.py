@@ -19,7 +19,8 @@ import torch
 import vpt_b200 as V
 from vpt_b200.scene import synthetic_env
 import oracle_ref
-from test_parity_gpu import flipped_fraction, make_kp, MAX_FLIPPED, needs_ref
+import reference_outputs
+from test_parity_gpu import flipped_fraction, make_kp, MAX_FLIPPED
 
 pytestmark = pytest.mark.gpu
 has_fill = os.path.exists(os.path.join(oracle_ref.REF_DIR, "texture_kernels_ref.cubin"))
@@ -36,17 +37,20 @@ def scene_of(vol):
     return V.Scene([vol.instance()], env=synthetic_env(512, 256), keep=[vol])
 
 
-@needs_ref
-@pytest.mark.skipif(not has_fill, reason="oracle/_ref/texture_kernels_ref.cubin not built")
-def test_procedural_fill_against_reference_fill_kernel():
+def test_procedural_fill_against_reference_fill_kernel(request):
     dims = (70, 52, 44)                                       # ragged: not multiples of the reference's 8x8x8 blocks
     vol = V.Volume.procedural(dims, scale=0.1, seed=123)
-    ref = torch.full((dims[0] * dims[1] * dims[2],), -7.0, dtype=torch.float32, device="cuda")
-    oracle_ref.RefOracle().fill_volume(ref.data_ptr(), dims, scale=0.1, noise_type=0)
-    torch.cuda.synchronize()
-    a = vol.dense.cpu().numpy(); b = ref.cpu().numpy()
+
+    def reference():
+        ref = torch.full((dims[0] * dims[1] * dims[2],), -7.0, dtype=torch.float32, device="cuda")
+        oracle_ref.RefOracle().fill_volume(ref.data_ptr(), dims, scale=0.1, noise_type=0)
+        torch.cuda.synchronize()
+        return dict(fill=ref)
+    R = reference_outputs.load(request, reference, live=oracle_ref.available() and has_fill)
+    full = vol.dense.cpu().numpy()
+    a = R.pick("fill", full); b = R.want("fill")
     print(f"reference fill: {int((b == -7.0).sum())} of {b.size} voxels untouched, finite {bool(np.isfinite(b).all())}, range [{np.nanmin(b):.3g}, {np.nanmax(b):.3g}]")
-    assert np.isfinite(a).all() and a.min() < -0.3 and a.max() > 0.3, "Perlin noise spans negative and positive densities (quirk Q10)"
+    assert np.isfinite(full).all() and full.min() < -0.3 and full.max() > 0.3, "Perlin noise spans negative and positive densities (quirk Q10)"
     print(f"fill: max |ours - reference| = {np.abs(a - b).max():.3g} (jitter bound ~ {0.1 / min(dims) * 2:.3g}), corr {np.corrcoef(a, b)[0, 1]:.6f}")
     # the reference jitters every sample position with an UNINITIALISED curand state (quirk Q14; its -O3 build does not even run): the
     # -G build used here draws some jitter, ours draws none -- the fields agree to the jitter's reach (~2 * scale / dim) and correlate to 1e-5
@@ -122,19 +126,22 @@ def test_software_filter_against_texture_unit(perlin):
     assert out[4 * prod] < 1e-6 and out[4 * prod + 2] / out[4 * prod + 3] > 0.99
 
 
-@needs_ref
-def test_parity_mode_on_the_procedural_volume_against_reference(perlin):
+def test_parity_mode_on_the_procedural_volume_against_reference(request, perlin):
     """tex3D path, negative densities included: per-seed parity with the reference kernel."""
     scene = scene_of(perlin)
     kw = dict(ray_depth=3, volume_depth=2)
-    mine = V.Renderer(scene, 320, 200, kp=make_kp(**kw)); ref = V.Renderer(scene, 320, 200, kp=make_kp(**kw), cam=mine.cam)
-    orc = oracle_ref.RefOracle()
-    ref.params.p_oct.value = orc.build_octree(scene.h_volumes, 1)
-    scene.reset_blue_noise(); orc.render(ref, 3)
+    mine = V.Renderer(scene, 320, 200, kp=make_kp(**kw))
+
+    def reference():
+        ref = V.Renderer(scene, 320, 200, kp=make_kp(**kw), cam=mine.cam)
+        orc = oracle_ref.RefOracle()
+        ref.params.p_oct.value = orc.build_octree(scene.h_volumes, 1)
+        scene.reset_blue_noise(); orc.render(ref, 3)
+        return dict(accum=ref.buffers.accum, mean=float(ref.buffers.accum.mean()))
+    R = reference_outputs.load(request, reference)
     scene.reset_blue_noise(); mine.render(3); torch.cuda.synchronize()
-    want = ref.buffers.accum.cpu().numpy()
-    assert float(want.mean()) > 1e-3
-    assert flipped_fraction(mine.buffers.accum.cpu().numpy(), want) <= MAX_FLIPPED
+    assert float(R.want("mean")) > 1e-3
+    assert flipped_fraction(R.pick("accum", mine.buffers.accum), R.want("accum")) <= MAX_FLIPPED
 
 
 def test_fast_mode_statistics_against_parity_mode(perlin):
@@ -158,38 +165,41 @@ def test_fast_mode_statistics_against_parity_mode(perlin):
     assert flipped_fraction(fast.buffers.depth.cpu().numpy()[:, None], par.buffers.depth.cpu().numpy()[:, None]) <= MAX_FLIPPED
 
 
-@needs_ref
-def test_fast_mode_converged_error_within_reference_noise_floor(perlin):
+def test_fast_mode_converged_error_within_reference_noise_floor(request, perlin):
     """SURVEY 8(c): converged (64 spp) RMSE of fast mode against the reference <= 1.1 x the reference-vs-reference RMSE obtained
     with a different `iteration` base (another set of Philox streams)."""
     scene = scene_of(perlin)
     W, H, P = 200, 120, 64
     kw = dict(ray_depth=2)
     fast = V.Renderer(scene, W, H, kp=make_kp(**kw)); fast.set_brick_volume(perlin)
-    ra = V.Renderer(scene, W, H, kp=make_kp(**kw), cam=fast.cam); rb = V.Renderer(scene, W, H, kp=make_kp(**kw), cam=fast.cam)
-    orc = oracle_ref.RefOracle()
-    root = orc.build_octree(scene.h_volumes, 1)
-    ra.params.p_oct.value = root; rb.params.p_oct.value = root
-    scene.reset_blue_noise(); fast.render(P)
-    scene.reset_blue_noise(); orc.render(ra, P)
-    # second reference run on other random streams: the passes that would be iterations 500 .. 500+P-1 (curand offset =
-    # iteration * 4096), each rendered into a zeroed accumulator so that accum = value / (iteration + 1), averaged by hand
-    acc = torch.zeros_like(rb.buffers.accum)
-    scene.reset_blue_noise()
-    for p in range(P):
-        rb.buffers.accum.zero_()
-        rb.kp.iteration = 500 + p                                           # < max_interactions (1000): still sampling
-        orc.launch(rb.params.array, W, H, orc.NOBN); orc.bn_advance(rb.kp)
+
+    def reference():
+        ra = V.Renderer(scene, W, H, kp=make_kp(**kw), cam=fast.cam); rb = V.Renderer(scene, W, H, kp=make_kp(**kw), cam=fast.cam)
+        orc = oracle_ref.RefOracle()
+        root = orc.build_octree(scene.h_volumes, 1)
+        ra.params.p_oct.value = root; rb.params.p_oct.value = root
+        scene.reset_blue_noise(); orc.render(ra, P)
+        # second reference run on other random streams: the passes that would be iterations 500 .. 500+P-1 (curand offset =
+        # iteration * 4096), each rendered into a zeroed accumulator so that accum = value / (iteration + 1), averaged by hand
+        acc = torch.zeros_like(rb.buffers.accum)
+        scene.reset_blue_noise()
+        for p in range(P):
+            rb.buffers.accum.zero_()
+            rb.kp.iteration = 500 + p                                       # < max_interactions (1000): still sampling
+            orc.launch(rb.params.array, W, H, orc.NOBN); orc.bn_advance(rb.kp)
+            torch.cuda.synchronize()
+            acc += rb.buffers.accum * float(500 + p + 1)
+        acc /= P
         torch.cuda.synchronize()
-        acc += rb.buffers.accum * float(500 + p + 1)
-    acc /= P
-    torch.cuda.synchronize()
-    a = ra.buffers.accum.cpu().numpy(); f = fast.buffers.accum.cpu().numpy(); b = acc.cpu().numpy()
+        return dict(accum=ra.buffers.accum, other_streams=acc, mean=float(ra.buffers.accum.mean()))
+    R = reference_outputs.load(request, reference)
+    scene.reset_blue_noise(); fast.render(P); torch.cuda.synchronize()
+    a = R.want("accum"); f = R.pick("accum", fast.buffers.accum); b = R.want("other_streams")
     rmse = lambda x, y: float(np.sqrt(np.mean((x - y) ** 2)))
     floor, err = rmse(b, a), rmse(f, a)
     print(f"converged {P} spp: RMSE fast-vs-reference {err:.4g}, reference-vs-reference (other streams) {floor:.4g}")
     assert floor > 0 and err <= 1.1 * floor
-    assert abs(float(f.mean()) - float(a.mean())) <= 0.01 * float(a.mean())
+    assert abs(float(fast.buffers.accum.mean()) - float(R.want("mean"))) <= 0.01 * float(R.want("mean"))
 
 
 def test_fast_mode_refuses_what_it_does_not_implement(perlin):

@@ -1,6 +1,7 @@
 """GPU parity tests: the sm_100a wavefront path (through the C ABI) against
   (1) the committed golden fixtures -- outputs of the reference's own kernel (tests/golden/make_golden.py), and
-  (2) when oracle/_ref travelled with the snapshot, the reference kernel executed live on the same parameter block.
+  (2) the reference kernel on the same parameter block: executed live where oracle/_ref was built, else its outputs as
+      recorded under tests/golden/reference (tests/reference_outputs.py).
 
 Tolerance (stated once, used everywhere): per channel |d| <= 1e-5 + 1e-4*|ref| on >= 99.9 % of the pixels; the rest
 are counted as decision-flipped pixels (chaotic estimator, SURVEY 8(c)).  In practice 0 pixels differ.
@@ -18,6 +19,7 @@ import torch
 import vpt_b200 as V
 from vpt_b200.scene import synthetic_env
 import oracle_ref
+import reference_outputs
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
@@ -72,7 +74,6 @@ def test_against_reference_golden(dragon, name):
 needs_ref = pytest.mark.skipif(not oracle_ref.available(), reason="oracle/_ref (reference kernel build) not in this snapshot")
 
 
-@needs_ref
 @pytest.mark.parametrize("cfg", [
     dict(W=256, H=256, passes=1, kp=dict(ray_depth=1)),                                   # BASELINE config 1 shape (HDRI env)
     dict(W=512, H=512, passes=1, kp=dict(ray_depth=1)),                                   # BASELINE config 1 resolution
@@ -81,38 +82,64 @@ needs_ref = pytest.mark.skipif(not oracle_ref.available(), reason="oracle/_ref (
     dict(W=200, H=120, passes=2, kp=dict(ray_depth=2, density_mult=6.0, tr_depth=0.5, sun_mult=3.0)),
     dict(W=33, H=17, passes=2, kp=dict(ray_depth=2)),                                     # tiny / not a multiple of any tile
 ])
-def test_live_against_reference_kernel(dragon, cfg):
+def test_live_against_reference_kernel(request, dragon, cfg):
     scene = make_scene(dragon)
     mine = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**cfg["kp"]))
-    ref = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**cfg["kp"]), cam=mine.cam)
-    orc = oracle_ref.RefOracle()
-    ref.params.p_oct.value = orc.build_octree(scene.h_volumes, 1)
-    scene.reset_blue_noise(); orc.render(ref, cfg["passes"]); bn_ref = scene.d_blue_noise.clone()
+
+    def reference():
+        ref = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**cfg["kp"]), cam=mine.cam)
+        orc = oracle_ref.RefOracle()
+        ref.params.p_oct.value = orc.build_octree(scene.h_volumes, 1)
+        scene.reset_blue_noise(); orc.render(ref, cfg["passes"])
+        return dict(accum=ref.buffers.accum, depth=ref.buffers.depth, blue_noise=scene.d_blue_noise, iteration=ref.kp.iteration)
+    R = reference_outputs.load(request, reference, exact=("blue_noise",))
     scene.reset_blue_noise(); mine.render(cfg["passes"]); torch.cuda.synchronize()
-    assert flipped_fraction(mine.buffers.accum.cpu().numpy(), ref.buffers.accum.cpu().numpy()) <= MAX_FLIPPED
-    assert flipped_fraction(mine.buffers.depth.cpu().numpy()[:, None], ref.buffers.depth.cpu().numpy()[:, None]) <= MAX_FLIPPED
-    assert torch.equal(scene.d_blue_noise, bn_ref)
-    assert mine.kp.iteration == ref.kp.iteration == cfg["passes"]
+    assert flipped_fraction(R.pick("accum", mine.buffers.accum), R.want("accum")) <= MAX_FLIPPED
+    assert flipped_fraction(R.pick("depth", mine.buffers.depth)[:, None], R.want("depth")[:, None]) <= MAX_FLIPPED
+    assert R.same("blue_noise", scene.d_blue_noise)
+    assert mine.kp.iteration == int(R.want("iteration")) == cfg["passes"]
 
 
-@needs_ref
-def test_point_lights_and_sphere_against_reference(dragon):
+def test_point_lights_and_sphere_against_reference(request, dragon):
     lights = [((9.0, 6.0, 2.0), (1.0, 0.8, 0.6), 40.0), ((-2.0, 3.0, 8.0), (0.5, 0.7, 1.0), 25.0), ((4.0, 9.0, 3.0), (1.0, 1.0, 1.0), 10.0)]
     scene = make_scene(dragon, lights=lights)
     # put the reference sphere where rays actually hit it: next to the dragon
     sp = scene.h_sphere; sp.center = V.f3(4.0, 6.5, 3.0); sp.radius = 1.2; sp.roughness = 0.7; sp.color = V.f3(0.8, 0.6, 0.3)
     scene.d_sphere.copy_(torch.frombuffer(bytearray(bytes(sp)), dtype=torch.uint8))
     kw = dict(ray_depth=3, volume_depth=2)
-    mine = V.Renderer(scene, 256, 160, kp=make_kp(**kw)); ref = V.Renderer(scene, 256, 160, kp=make_kp(**kw), cam=mine.cam)
-    orc = oracle_ref.RefOracle()
-    scene.reset_blue_noise(); orc.render(ref, 2)
+    mine = V.Renderer(scene, 256, 160, kp=make_kp(**kw))
+
+    def reference():
+        ref = V.Renderer(scene, 256, 160, kp=make_kp(**kw), cam=mine.cam)
+        scene.reset_blue_noise(); oracle_ref.RefOracle().render(ref, 2)
+        return dict(accum=ref.buffers.accum, mean=float(ref.buffers.accum.mean()))
+    R = reference_outputs.load(request, reference)
     scene.reset_blue_noise(); mine.render(2); torch.cuda.synchronize()
-    assert float(ref.buffers.accum.mean()) > 0
-    assert flipped_fraction(mine.buffers.accum.cpu().numpy(), ref.buffers.accum.cpu().numpy()) <= MAX_FLIPPED
+    assert float(R.want("mean")) > 0
+    assert flipped_fraction(R.pick("accum", mine.buffers.accum), R.want("accum")) <= MAX_FLIPPED
 
 
-@needs_ref
-def test_instanced_scene_and_octree_bit_exact(dragon):
+def octree_arrays(tree):
+    """An octree read with vpt_octree_read (node number -> OCTNode) as flat arrays; the host-built root (node 0) carries
+    no voxel size, depth or child flag."""
+    paths = sorted(tree)
+    n = [tree[p].num_volumes for p in paths]
+    return dict(paths=np.array(paths, dtype=np.int32), num_volumes=np.array(n, dtype=np.int32),
+                vol_indices=np.array([v for p in paths for v in tree[p].vol_indices[:tree[p].num_volumes]], dtype=np.int32),
+                bbox=np.array([np.frombuffer(bytes(tree[p].bbox), dtype=np.float32) for p in paths], dtype=np.float32),
+                extinction=np.array([(tree[p].max_extinction, tree[p].min_extinction) for p in paths], dtype=np.float32),
+                node=np.array([(tree[p].voxel_size, tree[p].depth, tree[p].has_children) if p else (0, 0, 0) for p in paths], dtype=np.float32))
+
+
+OCTREE_ARRAYS = ("paths", "num_volumes", "vol_indices", "bbox", "extinction", "node")
+
+
+def assert_octree_equals_reference(R, tree):
+    for k, a in octree_arrays(tree).items():
+        assert R.same(k, a), k
+
+
+def test_instanced_scene_and_octree_bit_exact(request, dragon):
     """8 rotated / scaled instances: my parallel octree build vs the reference's device-heap recursion, node by
     node (bbox, volume lists, extinctions bit-exact), then the render on both octrees."""
     rng = np.random.RandomState(7)
@@ -121,42 +148,50 @@ def test_instanced_scene_and_octree_bit_exact(dragon):
         q = rng.randn(4); q /= np.linalg.norm(q)
         inst.append(dragon.instance(pos=tuple(rng.uniform(-6, 6, 3)), quat=tuple(q), scale=float(rng.uniform(0.6, 1.4))))
     scene = make_scene(dragon, instances=inst)
-    orc = oracle_ref.RefOracle()
-    ref_root = orc.build_octree(scene.h_volumes, len(inst))
-
-    def read_tree(root):
-        nodes = (V.OCTNode * 585)(); ex = (C.c_int * 585)()
-        V._native.check(V.lib.vpt_octree_read(root, nodes, ex), None, "vpt_octree_read")
-        return {j: nodes[j] for j in range(585) if ex[j]}
-    mine_t, ref_t = read_tree(scene.d_oct_root), read_tree(ref_root)
-    assert mine_t.keys() == ref_t.keys() and len(mine_t) > 9
-    for path in ref_t:
-        a, b = mine_t[path], ref_t[path]
-        assert a.num_volumes == b.num_volumes, path
-        assert list(a.vol_indices[:a.num_volumes]) == list(b.vol_indices[:b.num_volumes]), path
-        assert bytes(a.bbox) == bytes(b.bbox), path
-        assert (a.max_extinction, a.min_extinction) == (b.max_extinction, b.min_extinction), path
-        if path: assert a.voxel_size == b.voxel_size and a.depth == b.depth and a.has_children == b.has_children, path   # path = node number; 0 is the host-built root
     kw = dict(ray_depth=2)
-    mine = V.Renderer(scene, 256, 128, kp=make_kp(**kw)); ref = V.Renderer(scene, 256, 128, kp=make_kp(**kw), cam=mine.cam)
-    ref.params.p_oct.value = ref_root
-    scene.reset_blue_noise(); orc.render(ref, 2)
+    mine = V.Renderer(scene, 256, 128, kp=make_kp(**kw))
+
+    def reference():
+        orc = oracle_ref.RefOracle()
+        ref_root = orc.build_octree(scene.h_volumes, len(inst))
+        ref = V.Renderer(scene, 256, 128, kp=make_kp(**kw), cam=mine.cam)
+        ref.params.p_oct.value = ref_root
+        scene.reset_blue_noise(); orc.render(ref, 2)
+        return dict(octree_arrays(read_tree(ref_root)), accum=ref.buffers.accum)
+    R = reference_outputs.load(request, reference, exact=OCTREE_ARRAYS)
+    mine_t = read_tree(scene.d_oct_root)
+    assert len(mine_t) > 9
+    assert_octree_equals_reference(R, mine_t)
     scene.reset_blue_noise(); mine.render(2); torch.cuda.synchronize()
-    assert flipped_fraction(mine.buffers.accum.cpu().numpy(), ref.buffers.accum.cpu().numpy()) <= MAX_FLIPPED
+    assert flipped_fraction(R.pick("accum", mine.buffers.accum), R.want("accum")) <= MAX_FLIPPED
 
 
-@needs_ref
-def test_instance_transform_matches_reference_mat4_algebra(dragon):
+def read_tree(root):
+    nodes = (V.OCTNode * 585)(); ex = (C.c_int * 585)()
+    V._native.check(V.lib.vpt_octree_read(root, nodes, ex), None, "vpt_octree_read")
+    return {j: nodes[j] for j in range(585) if ex[j]}
+
+
+def test_instance_transform_matches_reference_mat4_algebra(request, dragon):
     from vpt_b200.scene import instance_xform
-    orc = oracle_ref.RefOracle()
     rng = np.random.RandomState(3)
     base = np.array([[dragon.rec.xform[a][b] for b in range(4)] for a in range(4)], dtype=np.float32)
     base[0][3], base[1][3], base[2][3] = 0.3, -0.2, 0.1
+    args = []
     for _ in range(20):
         q = rng.randn(4).astype(np.float32); pos = rng.uniform(-50, 50, 3).astype(np.float32); s = np.float32(rng.uniform(0.2, 3))
-        out = (C.c_float * 16)()
-        orc.lib.vptref_instance_xform(V._native.fvec(base.reshape(-1)), V._native.fvec(pos), V._native.fvec(q), float(s), out)
-        assert np.array_equal(np.array(list(out), dtype=np.float32).reshape(4, 4), instance_xform(base, pos, q, s))
+        args.append((pos, q, s))
+
+    def reference():
+        orc = oracle_ref.RefOracle()
+        xf = []
+        for pos, q, s in args:
+            out = (C.c_float * 16)()
+            orc.lib.vptref_instance_xform(V._native.fvec(base.reshape(-1)), V._native.fvec(pos), V._native.fvec(q), float(s), out)
+            xf.append(np.array(list(out), dtype=np.float32).reshape(4, 4))
+        return dict(xforms=np.stack(xf))
+    R = reference_outputs.load(request, reference)
+    assert R.same("xforms", np.stack([instance_xform(base, pos, q, s) for pos, q, s in args]).astype(np.float32))
 
 
 def _big_asset(name):
@@ -198,8 +233,7 @@ def test_colored_smoke_against_reference():
     assert flipped_fraction(mine.buffers.accum.cpu().numpy(), a) <= MAX_FLIPPED
 
 
-@needs_ref
-def test_many_instances_against_reference(dragon):
+def test_many_instances_against_reference(request, dragon):
     """BASELINE config 5 shape (instanced dragon through the octree's leaf lists) at the size the oracle finishes quickly."""
     rng = np.random.RandomState(11)
     inst = []
@@ -208,17 +242,46 @@ def test_many_instances_against_reference(dragon):
         inst.append(dragon.instance(pos=tuple(rng.uniform(-25, 25, 3)), quat=tuple(q), scale=float(rng.uniform(0.7, 1.3))))
     scene = make_scene(dragon, instances=inst)
     kw = dict(ray_depth=2)
-    mine = V.Renderer(scene, 256, 144, kp=make_kp(**kw)); ref = V.Renderer(scene, 256, 144, kp=make_kp(**kw), cam=mine.cam)
-    orc = oracle_ref.RefOracle()
-    scene.reset_blue_noise(); orc.render(ref, 1)
+    mine = V.Renderer(scene, 256, 144, kp=make_kp(**kw))
+
+    def reference():
+        ref = V.Renderer(scene, 256, 144, kp=make_kp(**kw), cam=mine.cam)
+        scene.reset_blue_noise(); oracle_ref.RefOracle().render(ref, 1)
+        return dict(accum=ref.buffers.accum, mean=float(ref.buffers.accum.mean()))
+    R = reference_outputs.load(request, reference)
     scene.reset_blue_noise(); mine.render(1); torch.cuda.synchronize()
-    assert float(ref.buffers.accum.mean()) > 1e-4
-    assert flipped_fraction(mine.buffers.accum.cpu().numpy(), ref.buffers.accum.cpu().numpy()) <= MAX_FLIPPED
+    assert float(R.want("mean")) > 1e-4
+    assert flipped_fraction(R.pick("accum", mine.buffers.accum), R.want("accum")) <= MAX_FLIPPED
 
 
-# ---- size-independent properties at the BASELINE resolution (no oracle needed) ------------------------------------
-@needs_ref
-@pytest.mark.skipif(not os.path.exists(os.path.join(oracle_ref.REF_DIR, "atmo", "atmosphere_kernels.ptx")), reason="oracle/_ref/atmo not built")
+# ---- the sky look-up tables: the reference's own precompute (live only) and this library's ----------------------------
+SKY_TABLES = ("reference", "own")
+_OWN_SKY = {}
+
+
+def sky_tables(scene, source, luminance=0):
+    """Hand `scene` the four sky look-up textures of one precompute, default options otherwise: "reference" (the reference's
+    own atmosphere::init, oracle/_ref) or "own" (this library's).  Both kernels then read the same textures."""
+    if source == "reference":
+        oracle_ref.RefOracle().atmosphere_init(scene.atmos, luminance=luminance)
+    else:
+        if luminance not in _OWN_SKY:
+            _OWN_SKY[luminance] = V.Atmosphere(luminance=luminance)
+        _OWN_SKY[luminance].apply(scene.atmos)
+
+
+def sky_sources(R):
+    """The table sources a test compares on: both where the reference runs live; its recorded frames on this library's tables otherwise."""
+    return SKY_TABLES if R.live else ("own",)
+
+
+def live_only_keys(*names):
+    return tuple(f"reference.{n}" for n in names)
+
+
+has_ref_atmo = os.path.exists(os.path.join(oracle_ref.REF_DIR, "atmo", "atmosphere_kernels.ptx"))
+
+
 @pytest.mark.parametrize("cfg", [
     dict(W=512, H=512, passes=1, elevation=30.0, kp=dict(ray_depth=1)),                          # BASELINE config 1 literally (env type 0)
     dict(W=320, H=200, passes=3, elevation=4.0, kp=dict(ray_depth=20, sky_mult=2.0)),            # low sun, multi-pass, deeper paths
@@ -226,24 +289,37 @@ def test_many_instances_against_reference(dragon):
     dict(W=256, H=128, passes=1, elevation=45.0, luminance=1, kp=dict(ray_depth=2)),             # APPROXIMATE luminance mode
     dict(W=256, H=128, passes=1, elevation=45.0, luminance=2, kp=dict(ray_depth=2)),             # PRECOMPUTED luminance mode
 ])
-def test_precomputed_sky_environment_against_reference(dragon, cfg):
-    """environment_type == 0: both kernels read the SAME look-up textures, produced by the reference's own precompute."""
+def test_precomputed_sky_environment_against_reference(request, dragon, cfg):
+    """environment_type == 0: both kernels read the SAME look-up textures, produced by the reference's own precompute and by
+    this library's."""
     scene = make_scene(dragon)
-    orc = oracle_ref.RefOracle()
-    orc.atmosphere_init(scene.atmos, luminance=cfg.get("luminance", 0))
     kw = dict(environment_type=0, elevation=cfg["elevation"], **cfg["kp"])
     cam = scene.frame_camera(cfg["W"], cfg["H"], aperture=cfg.get("aperture", 0.0))
-    mine = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**kw), cam=cam)
-    ref = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**kw), cam=cam)
-    scene.reset_blue_noise(); orc.render(ref, cfg["passes"])
-    scene.reset_blue_noise(); mine.render(cfg["passes"]); torch.cuda.synchronize()
-    want = ref.buffers.accum.cpu().numpy(); got = mine.buffers.accum.cpu().numpy()
-    print(f"sky cfg {cfg}: reference mean {float(want.mean()):.6g}, ours {float(got.mean()):.6g}")
-    assert np.isfinite(want).all()
-    if not cfg.get("luminance"):
-        assert float(want.mean()) > 1e-3 and want.std() > 0, "the sky must actually light the frame"
-    assert flipped_fraction(got, want) <= MAX_FLIPPED
-    assert flipped_fraction(mine.buffers.depth.cpu().numpy()[:, None], ref.buffers.depth.cpu().numpy()[:, None]) <= MAX_FLIPPED
+    lum = cfg.get("luminance", 0)
+
+    def reference():
+        out = {}
+        for src in SKY_TABLES:
+            sky_tables(scene, src, lum)
+            ref = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**kw), cam=cam)
+            scene.reset_blue_noise(); oracle_ref.RefOracle().render(ref, cfg["passes"])
+            a = ref.buffers.accum.cpu().numpy()
+            out.update({f"{src}.accum": a, f"{src}.depth": ref.buffers.depth,
+                        f"{src}.stats": np.array([np.isfinite(a).all(), a.mean(), a.std()], dtype=np.float64)})
+        return out
+    R = reference_outputs.load(request, reference, live=oracle_ref.available() and has_ref_atmo, live_only=live_only_keys("accum", "depth", "stats"))
+    for src in sky_sources(R):
+        sky_tables(scene, src, lum)
+        mine = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**kw), cam=cam)
+        scene.reset_blue_noise(); mine.render(cfg["passes"]); torch.cuda.synchronize()
+        want = R.want(f"{src}.accum"); got = R.pick(f"{src}.accum", mine.buffers.accum)
+        finite, mean, std = R.want(f"{src}.stats")
+        print(f"sky cfg {cfg}, {src} tables: reference mean {mean:.6g}, ours {float(mine.buffers.accum.mean()):.6g}")
+        assert finite
+        if not lum:
+            assert mean > 1e-3 and std > 0, "the sky must actually light the frame"
+        assert flipped_fraction(got, want) <= MAX_FLIPPED
+        assert flipped_fraction(R.pick(f"{src}.depth", mine.buffers.depth)[:, None], R.want(f"{src}.depth")[:, None]) <= MAX_FLIPPED
 
 
 def _sky_power_table(res=180, sun_az=2.0, sun_el=1.0):
@@ -254,8 +330,6 @@ def _sky_power_table(res=180, sun_az=2.0, sun_el=1.0):
     return (0.05 + np.sin(el) * (1.2 + np.cos(az - sun_az)) * (0.3 + np.exp(-4.0 * (el - sun_el) ** 2))).astype(np.float32)
 
 
-@needs_ref
-@pytest.mark.skipif(not os.path.exists(os.path.join(oracle_ref.REF_DIR, "atmo", "atmosphere_kernels.ptx")), reason="oracle/_ref/atmo not built")
 @pytest.mark.parametrize("cfg", [
     dict(W=256, H=160, passes=2, env=1, kp=dict(ray_depth=8)),                                    # HDRI sky estimator (uniform sphere + HG MIS)
     dict(W=256, H=160, passes=2, env=1, kp=dict(ray_depth=100, phase_g1=0.6, density_mult=3.0)),  # cfg 2's "true multiple scattering" variant
@@ -263,35 +337,47 @@ def _sky_power_table(res=180, sun_az=2.0, sun_el=1.0):
     dict(W=200, H=120, passes=1, env=1, lights=True, kp=dict(ray_depth=5, sky_mult=0.0)),         # point lights, sky class switched off
     dict(W=160, H=100, passes=1, env=1, sphere=True, aperture=0.15, kp=dict(ray_depth=4)),        # sphere in the way + thin lens
 ])
-def test_volumetric_path_integrator_against_reference(dragon, cfg):
+def test_volumetric_path_integrator_against_reference(request, dragon, cfg):
     """Kernel_params.integrator = 1 (reference vol_integrator): light-class selection, NEE per scatter, sky MIS, sky tail."""
     lights = [((9.0, 6.0, 2.0), (1.0, 0.8, 0.6), 40.0), ((-2.0, 3.0, 8.0), (0.5, 0.7, 1.0), 25.0)] if cfg.get("lights") else None
     scene = make_scene(dragon, lights=lights)
     if cfg.get("sphere"):
         sp = scene.h_sphere; sp.center = V.f3(6.0, 6.0, 5.0); sp.radius = 1.0
         scene.d_sphere.copy_(torch.frombuffer(bytearray(bytes(sp)), dtype=torch.uint8))
-    orc = oracle_ref.RefOracle()
-    orc.atmosphere_init(scene.atmos)
     tables = V.EnvTables(_sky_power_table())
     kw = dict(integrator=1, environment_type=cfg["env"], **cfg["kp"])
     cam = scene.frame_camera(cfg["W"], cfg["H"], aperture=cfg.get("aperture", 0.0))
-    mine = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**kw), cam=cam)
-    ref = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**kw), cam=cam)
-    tables.apply(mine.kp); tables.apply(ref.kp)
-    scene.reset_blue_noise(); orc.render(ref, cfg["passes"])
-    scene.reset_blue_noise(); mine.render(cfg["passes"]); torch.cuda.synchronize()
-    want = ref.buffers.accum.cpu().numpy(); got = mine.buffers.accum.cpu().numpy()
-    frac = flipped_fraction(got, want)
-    dfrac = flipped_fraction(mine.buffers.depth.cpu().numpy()[:, None], ref.buffers.depth.cpu().numpy()[:, None])
-    print(f"vol cfg {cfg}: ref mean {float(want.mean()):.6g} ours {float(got.mean()):.6g} flipped {frac:.3g} depth-flipped {dfrac:.3g}")
-    assert np.isfinite(want).all() and float(want.mean()) > 1e-3
-    # Measured: no pixel outside tolerance in any configuration.  With the tabulated sky (env 0) the sky model is also evaluated
-    # INSIDE the path, where the reference build contracts three ill-conditioned sums differently from its end-of-path call sites;
-    # vpt_atmosphere.cuh mirrors both orders (kInPath).  Before that 0.25 % of the pixels were off by up to 1 % (DESIGN.md section 5).
-    limit = 1e-4 if cfg["env"] == 0 else 0.0
-    assert frac <= limit and dfrac == 0.0
-    raw_m = mine.buffers.raw.cpu().numpy().reshape(-1, 4)[:, 3]; raw_r = ref.buffers.raw.cpu().numpy().reshape(-1, 4)[:, 3]
-    assert np.mean(np.abs(raw_m - raw_r) > 1e-5) <= MAX_FLIPPED
+
+    def reference():
+        out = {}
+        for src in SKY_TABLES:
+            sky_tables(scene, src)
+            ref = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**kw), cam=cam)
+            tables.apply(ref.kp)
+            scene.reset_blue_noise(); oracle_ref.RefOracle().render(ref, cfg["passes"])
+            a = ref.buffers.accum.cpu().numpy()
+            out.update({f"{src}.accum": a, f"{src}.depth": ref.buffers.depth, f"{src}.tr": ref.buffers.raw.reshape(-1, 4)[:, 3],
+                        f"{src}.stats": np.array([np.isfinite(a).all(), a.mean()], dtype=np.float64)})
+        return out
+    R = reference_outputs.load(request, reference, live=oracle_ref.available() and has_ref_atmo, live_only=live_only_keys("accum", "depth", "tr", "stats"))
+    for src in sky_sources(R):
+        sky_tables(scene, src)
+        mine = V.Renderer(scene, cfg["W"], cfg["H"], kp=make_kp(**kw), cam=cam)
+        tables.apply(mine.kp)
+        scene.reset_blue_noise(); mine.render(cfg["passes"]); torch.cuda.synchronize()
+        want = R.want(f"{src}.accum"); got = R.pick(f"{src}.accum", mine.buffers.accum)
+        frac = flipped_fraction(got, want)
+        dfrac = flipped_fraction(R.pick(f"{src}.depth", mine.buffers.depth)[:, None], R.want(f"{src}.depth")[:, None])
+        finite, mean = R.want(f"{src}.stats")
+        print(f"vol cfg {cfg}, {src} tables: ref mean {mean:.6g} ours {float(mine.buffers.accum.mean()):.6g} flipped {frac:.3g} depth-flipped {dfrac:.3g}")
+        assert finite and mean > 1e-3
+        # Measured: no pixel outside tolerance in any configuration.  With the tabulated sky (env 0) the sky model is also evaluated
+        # INSIDE the path, where the reference build contracts three ill-conditioned sums differently from its end-of-path call sites;
+        # vpt_atmosphere.cuh mirrors both orders (kInPath).  Before that 0.25 % of the pixels were off by up to 1 % (DESIGN.md section 5).
+        limit = 1e-4 if cfg["env"] == 0 else 0.0
+        assert frac <= limit and dfrac == 0.0
+        tr = R.pick(f"{src}.tr", mine.buffers.raw.reshape(-1, 4)[:, 3])
+        assert np.mean(np.abs(tr - R.want(f"{src}.tr")) > 1e-5) <= MAX_FLIPPED
     tables.destroy()
 
 
@@ -361,8 +447,7 @@ def test_unsupported_configurations_fail_loudly(dragon):
         r.render_pass()
 
 
-@needs_ref
-def test_ins_scene_file_end_to_end_against_reference(tmp_path):
+def test_ins_scene_file_end_to_end_against_reference(request, tmp_path):
     """SURVEY 8(f) N4: a `.ins` file is read by the library, instanced with the reference's transform algebra, rendered."""
     from vpt_b200.scene import scene_from_ins
     ins = tmp_path / "three.ins"
@@ -370,10 +455,15 @@ def test_ins_scene_file_end_to_end_against_reference(tmp_path):
     scene = scene_from_ins(str(ins), env=synthetic_env(512, 256), resolve=V.find_asset)
     assert len(scene.instances) == 3
     kw = dict(ray_depth=3, volume_depth=2)
-    mine = V.Renderer(scene, 320, 200, kp=make_kp(**kw)); ref = V.Renderer(scene, 320, 200, kp=make_kp(**kw), cam=mine.cam)
-    orc = oracle_ref.RefOracle()
-    ref.params.p_oct.value = orc.build_octree(scene.h_volumes, 3)
-    scene.reset_blue_noise(); orc.render(ref, 2)
+    mine = V.Renderer(scene, 320, 200, kp=make_kp(**kw))
+
+    def reference():
+        ref = V.Renderer(scene, 320, 200, kp=make_kp(**kw), cam=mine.cam)
+        orc = oracle_ref.RefOracle()
+        ref.params.p_oct.value = orc.build_octree(scene.h_volumes, 3)
+        scene.reset_blue_noise(); orc.render(ref, 2)
+        return dict(accum=ref.buffers.accum, mean=float(ref.buffers.accum.mean()))
+    R = reference_outputs.load(request, reference)
     scene.reset_blue_noise(); mine.render(2); torch.cuda.synchronize()
-    assert float(ref.buffers.accum.mean()) > 0
-    assert flipped_fraction(mine.buffers.accum.cpu().numpy(), ref.buffers.accum.cpu().numpy()) <= MAX_FLIPPED
+    assert float(R.want("mean")) > 0
+    assert flipped_fraction(R.pick("accum", mine.buffers.accum), R.want("accum")) <= MAX_FLIPPED

@@ -19,7 +19,9 @@ import torch
 import vpt_b200 as V
 from vpt_b200.scene import synthetic_env
 import oracle_ref
-from test_parity_gpu import flipped_fraction, make_kp, make_scene, MAX_FLIPPED, needs_ref, _big_asset, _sky_power_table
+import reference_outputs
+from test_parity_gpu import (flipped_fraction, make_kp, make_scene, MAX_FLIPPED, needs_ref, _big_asset, _sky_power_table, read_tree, octree_arrays,
+                             assert_octree_equals_reference, OCTREE_ARRAYS, SKY_TABLES, sky_tables, sky_sources)
 
 pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -38,23 +40,6 @@ def scattered(dragon, n, seed, spread):
         q = rng.randn(4); q /= np.linalg.norm(q)
         inst.append(dragon.instance(pos=tuple(rng.uniform(-spread, spread, 3)), quat=tuple(q), scale=float(rng.uniform(0.7, 1.3))))
     return inst
-
-
-def read_tree(root):
-    nodes = (V.OCTNode * 585)(); ex = (C.c_int * 585)()
-    V._native.check(V.lib.vpt_octree_read(root, nodes, ex), None, "vpt_octree_read")
-    return {j: nodes[j] for j in range(585) if ex[j]}
-
-
-def assert_trees_equal(mine_t, ref_t):
-    assert mine_t.keys() == ref_t.keys()
-    for path in ref_t:
-        a, b = mine_t[path], ref_t[path]
-        assert a.num_volumes == b.num_volumes, path
-        assert list(a.vol_indices[:a.num_volumes]) == list(b.vol_indices[:b.num_volumes]), path
-        assert bytes(a.bbox) == bytes(b.bbox), path
-        assert (a.max_extinction, a.min_extinction) == (b.max_extinction, b.min_extinction), path
-        if path: assert a.voxel_size == b.voxel_size and a.depth == b.depth and a.has_children == b.has_children, path
 
 
 # ---- the timed configuration, checked ------------------------------------------------------------------------------
@@ -122,62 +107,72 @@ def test_baseline_config3_volumetric_path_integrator_against_reference():
     tables.destroy()
 
 
-@needs_ref
-def test_unmodified_reference_kernel_equals_race_free_protocol_at_256(dragon):
+def test_unmodified_reference_kernel_equals_race_free_protocol_at_256(request, dragon):
     """SURVEY 8(c)(i): at 256x256 every thread of the unmodified kernel touches only its own blue-noise entry, so the kernel is
     race-free there.  It must equal the protocol every other test uses (nobn build + the reference's own update statements as a
     separate launch) bit for bit -- and this library."""
     scene = make_scene(dragon)
     kw = dict(ray_depth=3, volume_depth=2)
-    a = V.Renderer(scene, 256, 256, kp=make_kp(**kw)); b = V.Renderer(scene, 256, 256, kp=make_kp(**kw), cam=a.cam)
-    mine = V.Renderer(scene, 256, 256, kp=make_kp(**kw), cam=a.cam)
-    orc = oracle_ref.RefOracle()
-    root = orc.build_octree(scene.h_volumes, 1)
-    a.params.p_oct.value = root; b.params.p_oct.value = root
-    scene.reset_blue_noise(); orc.render(a, 4, race_free=False); bn_a = scene.d_blue_noise.clone()
-    scene.reset_blue_noise(); orc.render(b, 4, race_free=True); bn_b = scene.d_blue_noise.clone()
+    mine = V.Renderer(scene, 256, 256, kp=make_kp(**kw))
+
+    def reference():
+        a = V.Renderer(scene, 256, 256, kp=make_kp(**kw), cam=mine.cam); b = V.Renderer(scene, 256, 256, kp=make_kp(**kw), cam=mine.cam)
+        orc = oracle_ref.RefOracle()
+        root = orc.build_octree(scene.h_volumes, 1)
+        a.params.p_oct.value = root; b.params.p_oct.value = root
+        scene.reset_blue_noise(); orc.render(a, 4, race_free=False); bn_a = scene.d_blue_noise.clone()
+        scene.reset_blue_noise(); orc.render(b, 4, race_free=True); bn_b = scene.d_blue_noise.clone()
+        for name in ("accum", "depth", "raw", "display", "cost"):
+            assert torch.equal(getattr(a.buffers, name), getattr(b.buffers, name)), name
+        assert torch.equal(bn_a, bn_b)
+        return dict(accum=a.buffers.accum, blue_noise=bn_a)
+    R = reference_outputs.load(request, reference, exact=("blue_noise",))
     scene.reset_blue_noise(); mine.render(4); torch.cuda.synchronize()
-    for name in ("accum", "depth", "raw", "display", "cost"):
-        assert torch.equal(getattr(a.buffers, name), getattr(b.buffers, name)), name
-    assert torch.equal(bn_a, bn_b) and torch.equal(bn_a, scene.d_blue_noise)
-    assert flipped_fraction(mine.buffers.accum.cpu().numpy(), a.buffers.accum.cpu().numpy()) <= MAX_FLIPPED
+    assert R.same("blue_noise", scene.d_blue_noise)
+    assert flipped_fraction(R.pick("accum", mine.buffers.accum), R.want("accum")) <= MAX_FLIPPED
 
 
 # ---- instance acceleration build (row N1) --------------------------------------------------------------------------
-@needs_ref
 @pytest.mark.parametrize("n,spread", [(120, 25.0), (600, 40.0)])
-def test_octree_node_for_node_and_render_at_many_instances(dragon, n, spread):
+def test_octree_node_for_node_and_render_at_many_instances(request, dragon, n, spread):
     inst = scattered(dragon, n, 11 + n, spread)
     scene = make_scene(dragon, instances=inst)
-    orc = oracle_ref.RefOracle()
-    ref_root = orc.build_octree(scene.h_volumes, n)
-    ref_t = read_tree(ref_root)
-    assert_trees_equal(read_tree(scene.d_oct_root), ref_t)
+    kw = dict(ray_depth=2)
+    W, H = (256, 144) if n <= 120 else (192, 108)
+    mine = V.Renderer(scene, W, H, kp=make_kp(**kw))
+    foreign = None
+
+    def reference():
+        nonlocal foreign
+        orc = oracle_ref.RefOracle()
+        ref_root = orc.build_octree(scene.h_volumes, n)
+        ref = V.Renderer(scene, W, H, kp=make_kp(**kw), cam=mine.cam)
+        foreign = V.Renderer(scene, W, H, kp=make_kp(**kw), cam=mine.cam)
+        ref.params.p_oct.value = ref_root
+        foreign.params.p_oct.value = ref_root        # this library on the REFERENCE's pointer-linked octree (k_prepare_scene path)
+        scene.reset_blue_noise(); orc.render(ref, 1)
+        scene.reset_blue_noise(); foreign.render(1); torch.cuda.synchronize()
+        return dict(octree_arrays(read_tree(ref_root)), accum=ref.buffers.accum, mean=float(ref.buffers.accum.mean()))
+    R = reference_outputs.load(request, reference, exact=OCTREE_ARRAYS)
+    mine_t = read_tree(scene.d_oct_root)
+    assert_octree_equals_reference(R, mine_t)
     # the flat (CSR) tables the render kernels read carry the same leaf lists
     lists = scene.leaf_lists()
     for l in range(512):
         j = 73 + l
-        want = list(ref_t[j].vol_indices[:ref_t[j].num_volumes]) if j in ref_t else []
+        want = list(mine_t[j].vol_indices[:mine_t[j].num_volumes]) if j in mine_t else []
         assert lists[l] == want, l
     info = scene.octree_info()
     assert info["n"] == n and info["reference_layout"] and info["total_leaf_entries"] == sum(len(x) for x in lists)
-    kw = dict(ray_depth=2)
-    W, H = (256, 144) if n <= 120 else (192, 108)
-    mine = V.Renderer(scene, W, H, kp=make_kp(**kw)); ref = V.Renderer(scene, W, H, kp=make_kp(**kw), cam=mine.cam)
-    foreign = V.Renderer(scene, W, H, kp=make_kp(**kw), cam=mine.cam)
-    ref.params.p_oct.value = ref_root
-    foreign.params.p_oct.value = ref_root            # this library on the REFERENCE's pointer-linked octree (k_prepare_scene path)
-    scene.reset_blue_noise(); orc.render(ref, 1)
-    scene.reset_blue_noise(); mine.render(1)
-    scene.reset_blue_noise(); foreign.render(1); torch.cuda.synchronize()
-    assert float(ref.buffers.accum.mean()) > 1e-4
-    assert flipped_fraction(mine.buffers.accum.cpu().numpy(), ref.buffers.accum.cpu().numpy()) <= MAX_FLIPPED
-    for name in ("accum", "depth", "raw", "display"):
-        assert torch.equal(getattr(mine.buffers, name), getattr(foreign.buffers, name)), name
+    scene.reset_blue_noise(); mine.render(1); torch.cuda.synchronize()
+    assert float(R.want("mean")) > 1e-4
+    assert flipped_fraction(R.pick("accum", mine.buffers.accum), R.want("accum")) <= MAX_FLIPPED
+    if foreign is not None:
+        for name in ("accum", "depth", "raw", "display"):
+            assert torch.equal(getattr(mine.buffers, name), getattr(foreign.buffers, name)), name
 
 
-@needs_ref
-def test_more_than_600_instances_through_flat_tables(dragon):
+def test_more_than_600_instances_through_flat_tables(request, dragon):
     """BASELINE configs[4] shape: 1000 instances, beyond the reference's OCTNode capacity (quirk Q11).  No oracle can run this,
     so: 500 real instances, each followed by a GHOST twin (same transform, all-zero density grid).  A ghost adds exactly +0.0f to
     every density sum and leaves every node's occupancy, the root box and the majorant unchanged, so the 1000-instance frame must
@@ -202,42 +197,58 @@ def test_more_than_600_instances_through_flat_tables(dragon):
         assert l1000[l] == [x for i in l500[l] for x in (2 * i, 2 * i + 1)], l
     kw = dict(ray_depth=2, volume_depth=2)
     a = V.Renderer(s500, 256, 144, kp=make_kp(**kw)); b = V.Renderer(s1000, 256, 144, kp=make_kp(**kw), cam=a.cam)
-    ref = V.Renderer(s500, 256, 144, kp=make_kp(**kw), cam=a.cam)
-    orc = oracle_ref.RefOracle()
-    ref.params.p_oct.value = orc.build_octree(s500.h_volumes, 500)
-    s500.reset_blue_noise(); orc.render(ref, 2)
+
+    def reference():
+        ref = V.Renderer(s500, 256, 144, kp=make_kp(**kw), cam=a.cam)
+        orc = oracle_ref.RefOracle()
+        ref.params.p_oct.value = orc.build_octree(s500.h_volumes, 500)
+        s500.reset_blue_noise(); orc.render(ref, 2)
+        return dict(accum=ref.buffers.accum, mean=float(ref.buffers.accum.mean()))
+    R = reference_outputs.load(request, reference)
     s500.reset_blue_noise(); a.render(2)
     s1000.reset_blue_noise(); b.render(2); torch.cuda.synchronize()
-    assert float(ref.buffers.accum.mean()) > 1e-4
-    assert flipped_fraction(a.buffers.accum.cpu().numpy(), ref.buffers.accum.cpu().numpy()) <= MAX_FLIPPED
+    assert float(R.want("mean")) > 1e-4
+    assert flipped_fraction(R.pick("accum", a.buffers.accum), R.want("accum")) <= MAX_FLIPPED
     for name in ("accum", "depth", "raw", "display"):
         assert torch.equal(getattr(a.buffers, name), getattr(b.buffers, name)), name
     with pytest.raises(V.VptError):                      # no reference-layout nodes exist for > 600 instances
         read_tree(s1000.d_oct_root)
 
 
-@needs_ref
+BVH_ARRAYS = ("scene_bounds", "leaves", "leaf_boxes", "nodes", "node_boxes")
+
+
+def bvh_arrays(scene_bounds, bvh):
+    """A BVH read with read_bvh as flat arrays (the reference never writes the root's parent: stored as 0)."""
+    box = lambda b: np.frombuffer(bytes(b), dtype=np.float32)
+    return dict(scene_bounds=np.array(scene_bounds, dtype=np.float32),
+                leaves=np.array([(l["volIndex"], l["parent"]) for l in bvh["leaves"]], dtype=np.int64).reshape(-1, 2),
+                leaf_boxes=np.array([box(l["box"]) for l in bvh["leaves"]], dtype=np.float32).reshape(-1, 6),
+                nodes=np.array([(d["left"], d["right"], d["minId"], d["maxId"], d["parent"] if i else 0) for i, d in enumerate(bvh["nodes"])],
+                               dtype=np.int64).reshape(-1, 5),
+                node_boxes=np.array([box(d["box"]) for d in bvh["nodes"]], dtype=np.float32).reshape(-1, 6))
+
+
 @pytest.mark.parametrize("n,spread,dups", [(2, 5.0, 0), (3, 5.0, 0), (37, 12.0, 6), (120, 25.0, 0), (600, 40.0, 40)])
-def test_lbvh_bit_exact_against_reference_builder(dragon, n, spread, dups):
+def test_lbvh_bit_exact_against_reference_builder(request, dragon, n, spread, dups):
     """Karras LBVH (bvh_kernels.cu:253-453, 460-580): sorted instance ids, child / parent topology, node ranges and boxes.
     `dups` instances repeat an earlier transform exactly, so equal Morton codes exercise the (code, id) tie-break."""
     inst = scattered(dragon, n - dups, 100 + n, spread)
     inst += [inst[i % len(inst)] for i in range(dups)]
     scene = make_scene(dragon, instances=inst)
     mine = scene.build_bvh()
-    orc = oracle_ref.RefOracle()
-    dn, dl = C.c_void_p(0), C.c_void_p(0); sb = (C.c_float * 6)()
-    rc = orc.lib.vptref_build_bvh(C.cast(scene.h_volumes, C.c_void_p), n, C.byref(dn), C.byref(dl), sb)
-    assert rc == 0
-    ref = V.read_bvh(dn.value, dl.value, n)
-    assert list(sb) == mine["scene_bounds"]
-    assert [l["volIndex"] for l in ref["leaves"]] == mine["ids"] == [l["volIndex"] for l in mine["leaves"]]
+
+    def reference():
+        orc = oracle_ref.RefOracle()
+        dn, dl = C.c_void_p(0), C.c_void_p(0); sb = (C.c_float * 6)()
+        rc = orc.lib.vptref_build_bvh(C.cast(scene.h_volumes, C.c_void_p), n, C.byref(dn), C.byref(dl), sb)
+        assert rc == 0
+        return bvh_arrays(list(sb), V.read_bvh(dn.value, dl.value, n))
+    R = reference_outputs.load(request, reference, exact=BVH_ARRAYS)
+    assert mine["ids"] == [l["volIndex"] for l in mine["leaves"]]
     assert sorted(mine["ids"]) == list(range(n)) and mine["codes"] == sorted(mine["codes"]) and max(mine["codes"]) < (1 << 30)
-    for i, (a, b) in enumerate(zip(mine["leaves"], ref["leaves"])):
-        assert (a["parent"], a["box"]) == (b["parent"], b["box"]), ("leaf", i)
-    for i, (a, b) in enumerate(zip(mine["nodes"], ref["nodes"])):
-        assert (a["left"], a["right"], a["minId"], a["maxId"], a["box"]) == (b["left"], b["right"], b["minId"], b["maxId"], b["box"]), ("node", i)
-        if i: assert a["parent"] == b["parent"], ("node", i)           # the reference never writes the root's parent
+    for k, a in bvh_arrays(mine["scene_bounds"], mine).items():
+        assert R.same(k, a), k
     # the root's box is the scene box, every internal node covers its [minId, maxId] leaf range
     root_box = np.frombuffer(mine["nodes"][0]["box"], dtype=np.float32)
     assert list(root_box) == mine["scene_bounds"]
@@ -349,14 +360,27 @@ def test_peer_memory_exchange_with_three_shards_on_one_gpu(dragon):
 LEVEL_A = os.path.join(os.path.dirname(V.LIB_PATH), "volume_rt_kernel_b200.cubin")
 
 
-def _launch_candidate(orc, r, passes):
-    for _ in range(passes):                                       # main.cpp:1823-1829: cuLaunchKernel(grid (w/16+1, h/16+1), block (16,16), params[9]); ++iteration; sync
-        orc.launch(r.params.array, r.width, r.height, orc.CANDIDATE)
-        r.kp.iteration += 1
-    torch.cuda.synchronize()
+def level_a_launcher():
+    """launch(r, passes): the level (A) cubin loaded and launched with cuModuleLoad + cuModuleGetFunction("volume_rt_kernel") +
+    cuLaunchKernel, one synchronised launch per pass with ++iteration (main.cpp:1823-1829).  Where oracle/_ref was built the calls
+    are the oracle harness's own, the very ones that drive the reference kernel; elsewhere LevelAModule issues the same three."""
+    if oracle_ref.available():
+        orc = oracle_ref.RefOracle(); orc.load_kernels(); orc.load_candidate(LEVEL_A)
+
+        def launch(r, passes):
+            for _ in range(passes):
+                orc.launch(r.params.array, r.width, r.height, orc.CANDIDATE)
+                r.kp.iteration += 1
+            torch.cuda.synchronize()
+        return launch
+    mod = V.LevelAModule(LEVEL_A)
+
+    def launch(r, passes):
+        for _ in range(passes):
+            mod.launch(r, sync=True)
+    return launch
 
 
-@needs_ref
 @pytest.mark.skipif(not os.path.exists(LEVEL_A), reason="volume_rt_kernel_b200.cubin not built")
 @pytest.mark.parametrize("cfg", [
     dict(W=512, H=512, passes=1, kp=dict(ray_depth=1)),                                    # BASELINE configs[0] resolution (plumbing config)
@@ -369,51 +393,69 @@ def _launch_candidate(orc, r, passes):
     dict(W=200, H=120, passes=1, kp=dict(ray_depth=6, integrator=1), atmo=True),           # volumetric path integrator, HDRI sky estimator
     dict(W=200, H=120, passes=1, kp=dict(ray_depth=2, environment_type=0), atmo=True),     # precomputed sky environment
 ])
-def test_level_a_module_through_the_reference_loader(dragon, cfg):
-    """The cubin is loaded with the harness's cuModuleLoad + cuModuleGetFunction("volume_rt_kernel") -- the same two calls and the same
-    cuLaunchKernel line that drive the reference kernel -- on the REFERENCE's own pointer-linked octree, and must match the oracle."""
-    if cfg.get("atmo") and not has_atmo: pytest.skip("oracle/_ref/atmo not built")
+def test_level_a_module_through_the_reference_loader(request, dragon, cfg):
+    """The cubin is loaded with cuModuleLoad + cuModuleGetFunction("volume_rt_kernel") -- the same two calls and the same
+    cuLaunchKernel line that drive the reference kernel -- and must match the oracle.  Live it runs on the REFERENCE's own
+    pointer-linked octree; on the recorded outputs, on this library's octree in the same layout (node for node equal to the
+    reference's: test_octree_node_for_node_and_render_at_many_instances)."""
     lights = [((9.0, 6.0, 2.0), (1.0, 0.8, 0.6), 40.0), ((-2.0, 3.0, 8.0), (0.5, 0.7, 1.0), 25.0)] if cfg.get("lights") else None
     inst = scattered(dragon, cfg["instances"], 9, 6.0) if cfg.get("instances") else None
     scene = make_scene(dragon, lights=lights, instances=inst)
     if cfg.get("sphere"):
         sp = scene.h_sphere; sp.center = V.f3(4.0, 6.5, 3.0); sp.radius = 1.2; sp.roughness = 0.7; sp.color = V.f3(0.8, 0.6, 0.3)
         scene.d_sphere.copy_(torch.frombuffer(bytearray(bytes(sp)), dtype=torch.uint8))
-    orc = oracle_ref.RefOracle()
-    if cfg.get("atmo"): orc.atmosphere_init(scene.atmos)
-    orc.load_kernels(); orc.load_candidate(LEVEL_A)
     W, H, P = cfg["W"], cfg["H"], cfg["passes"]
     cam = scene.frame_camera(W, H, aperture=cfg.get("aperture", 0.0))
-    a = V.Renderer(scene, W, H, kp=make_kp(**cfg["kp"]), cam=cam); ref = V.Renderer(scene, W, H, kp=make_kp(**cfg["kp"]), cam=cam)
-    root = orc.build_octree(scene.h_volumes, len(scene.instances))
-    a.params.p_oct.value = root; ref.params.p_oct.value = root
-    scene.reset_blue_noise(); orc.render(ref, P, race_free=not cfg.get("unmodified")); bn_ref = scene.d_blue_noise.clone()
-    scene.reset_blue_noise(); _launch_candidate(orc, a, P)
-    want = ref.buffers.accum.cpu().numpy(); got = a.buffers.accum.cpu().numpy()
-    frac = flipped_fraction(got, want)
-    print(f"level A {cfg}: flipped {frac:.3g}, max |d| {np.abs(got - want).max():.3g}, ref mean {want.mean():.6g}")
-    assert float(want.mean()) > 1e-4 and frac <= MAX_FLIPPED
-    assert flipped_fraction(a.buffers.depth.cpu().numpy()[:, None], ref.buffers.depth.cpu().numpy()[:, None]) <= MAX_FLIPPED
-    assert torch.equal(scene.d_blue_noise, bn_ref), "blue-noise state after the passes"
-    assert float(a.buffers.cost.abs().max()) == 0.0
-    dm = a.buffers.display.cpu().numpy().view(np.uint8).reshape(-1, 4).astype(int)
-    dr = ref.buffers.display.cpu().numpy().view(np.uint8).reshape(-1, 4).astype(int)
-    assert np.abs(dm - dr).max() <= 1
-    assert a.kp.iteration == ref.kp.iteration == P
+    sources = SKY_TABLES if cfg.get("atmo") else ("hdri",)
+    ref_root = None
+
+    def reference():
+        nonlocal ref_root
+        orc = oracle_ref.RefOracle()
+        ref_root = orc.build_octree(scene.h_volumes, len(scene.instances))
+        out = {}
+        for src in sources:
+            if cfg.get("atmo"): sky_tables(scene, src)
+            ref = V.Renderer(scene, W, H, kp=make_kp(**cfg["kp"]), cam=cam)
+            ref.params.p_oct.value = ref_root
+            scene.reset_blue_noise(); orc.render(ref, P, race_free=not cfg.get("unmodified"))
+            out.update({f"{src}.accum": ref.buffers.accum, f"{src}.depth": ref.buffers.depth, f"{src}.display": ref.buffers.display,
+                        f"{src}.blue_noise": scene.d_blue_noise.clone(), f"{src}.mean": float(ref.buffers.accum.mean()), f"{src}.iteration": ref.kp.iteration})
+        return out
+    live = oracle_ref.available() and (has_atmo or not cfg.get("atmo"))
+    R = reference_outputs.load(request, reference, live=live, exact=tuple(f"{s}.blue_noise" for s in sources),
+                               live_only=tuple(f"reference.{k}" for k in ("accum", "depth", "display", "blue_noise", "mean", "iteration")))
+    launch = level_a_launcher()
+    for src in (sky_sources(R) if cfg.get("atmo") else sources):
+        if cfg.get("atmo"): sky_tables(scene, src)
+        a = V.Renderer(scene, W, H, kp=make_kp(**cfg["kp"]), cam=cam)
+        if ref_root is not None: a.params.p_oct.value = ref_root
+        scene.reset_blue_noise(); launch(a, P)
+        want = R.want(f"{src}.accum"); got = R.pick(f"{src}.accum", a.buffers.accum)
+        frac = flipped_fraction(got, want)
+        print(f"level A {cfg}, {src}: flipped {frac:.3g}, max |d| {np.abs(got - want).max():.3g}, ref mean {float(R.want(f'{src}.mean')):.6g}")
+        assert float(R.want(f"{src}.mean")) > 1e-4 and frac <= MAX_FLIPPED
+        assert flipped_fraction(R.pick(f"{src}.depth", a.buffers.depth)[:, None], R.want(f"{src}.depth")[:, None]) <= MAX_FLIPPED
+        assert R.same(f"{src}.blue_noise", scene.d_blue_noise), "blue-noise state after the passes"
+        assert float(a.buffers.cost.abs().max()) == 0.0
+        dm = R.pick(f"{src}.display", a.buffers.display).view(np.uint8).reshape(-1, 4).astype(int)
+        dr = R.want(f"{src}.display").view(np.uint8).reshape(-1, 4).astype(int)
+        assert np.abs(dm - dr).max() <= 1
+        assert a.kp.iteration == int(R.want(f"{src}.iteration")) == P
 
 
-@needs_ref
 @pytest.mark.skipif(not os.path.exists(LEVEL_A), reason="volume_rt_kernel_b200.cubin not built")
 def test_level_a_non_sampling_passes(dragon):
     """iteration >= max_interactions: buffers are only re-tonemapped; render == false: WHITE into the accumulator (:2248-2287)."""
     scene = make_scene(dragon)
-    orc = oracle_ref.RefOracle(); orc.load_kernels(); orc.load_candidate(LEVEL_A)
+    launch = level_a_launcher()
     a = V.Renderer(scene, 128, 64, kp=make_kp(ray_depth=1, max_interactions=2))
-    a.params.p_oct.value = orc.build_octree(scene.h_volumes, 1)
-    _launch_candidate(orc, a, 2); acc2 = a.buffers.accum.clone()
-    _launch_candidate(orc, a, 2)
+    if oracle_ref.available():
+        a.params.p_oct.value = oracle_ref.RefOracle().build_octree(scene.h_volumes, 1)
+    launch(a, 2); acc2 = a.buffers.accum.clone()
+    launch(a, 2)
     assert torch.equal(acc2, a.buffers.accum)
     b = V.Renderer(scene, 128, 64, kp=make_kp(ray_depth=1, render=0), cam=a.cam)
     b.params.p_oct.value = a.params.p_oct.value
-    _launch_candidate(orc, b, 1)
+    launch(b, 1)
     assert torch.equal(b.buffers.accum, torch.ones_like(b.buffers.accum))
