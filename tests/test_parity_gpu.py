@@ -27,8 +27,14 @@ RTOL, ATOL, MAX_FLIPPED = 1e-4, 1e-5, 1e-3
 
 
 def flipped_fraction(got, want):
+    """Fraction of the pixels (rows) with a channel outside the tolerance.  A non-finite value matches only the same value:
+    NaN against NaN, +Inf against +Inf, -Inf against -Inf; finite against non-finite is a flip."""
     got = np.asarray(got, dtype=np.float64); want = np.asarray(want, dtype=np.float64)
-    bad = np.abs(got - want) > ATOL + RTOL * np.abs(want)
+    with np.errstate(invalid="ignore"):
+        bad = np.abs(got - want) > ATOL + RTOL * np.abs(want)
+    fin_g, fin_w = np.isfinite(got), np.isfinite(want)
+    both = ~fin_g & ~fin_w
+    bad |= (fin_g != fin_w) | (both & ~((np.isnan(got) & np.isnan(want)) | (got == want)))
     if bad.ndim > 1:
         bad = bad.reshape(bad.shape[0] * bad.shape[1] if bad.ndim == 3 else bad.shape[0], -1).any(axis=1)
     return float(bad.mean())

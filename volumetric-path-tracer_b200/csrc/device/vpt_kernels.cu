@@ -249,6 +249,10 @@ k_generate(const FrameArgs fa)
 struct NoSky { int pad[4]; };
 struct PeerFlagPtrs { unsigned long long* p[kMaxPeers]; };
 
+// The guard's load of the previous frame, out of line: inlined, it costs the HDRI variant 5 registers (32 -> 37) for a branch
+// that finite samples never take.
+__device__ __noinline__ float3 stale_pixel(const float3* accum_buf, uint32_t lp) { return accum_buf[lp]; }
+
 template <int kSky>
 __global__ void __launch_bounds__(256)
 k_resolve(const FrameArgs fa, const typename std::conditional<kSky != 0, vpt_atmosphere, NoSky>::type atmo,
@@ -302,8 +306,9 @@ k_resolve(const FrameArgs fa, const typename std::conditional<kSky != 0, vpt_atm
             tr = fminf(tr, 1.0f);
             value = L;
         }
-        // NaN / Inf guard (:2263-2264)
-        if (any_nan(value) || any_inf(value)) value = accum;
+        // NaN / Inf guard (:2263-2264): the pixel as the buffer holds it.  At iteration 0 that is the previous frame, which
+        // `accum` was not loaded with; the load stays in this branch so finite samples do not pay for it
+        if (any_nan(value) || any_inf(value)) value = iteration == 0 ? stale_pixel(accum_buf, lp) : accum;
         if (isnan(tr) || isinf(tr)) tr = 1.0f;
 
         float aof = 1 / cam.lens_radius;

@@ -61,7 +61,8 @@ VPT_DEV void resolve_pixel(const FrameArgs& fa, const vpt_atmosphere& atmo, uint
         tr = fminf(tr, 1.0f);
         value = L;
     }
-    if (any_nan(value) || any_inf(value)) value = accum;
+    // NaN / Inf guard (:2263): the pixel as the buffer holds it -- at iteration 0 the previous frame, which `accum` was not loaded with
+    if (any_nan(value) || any_inf(value)) value = iteration == 0 ? accum_buf[idx] : accum;
     if (isnan(tr) || isinf(tr)) tr = 1.0f;
 
     float aof = 1 / cam.lens_radius;
